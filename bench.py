@@ -10,6 +10,7 @@ controls + merit downloaded every step).  `--impl reference` times the CPU oracl
 host cores (the Julia reference cannot run here: no Julia in the image).
 
     python bench.py --gpus 1 --steps 20 --warmup 3
+    python bench.py --gpus 1 --steps 20 --warmup 3 --dump-outputs DIR     # also writes the last timed step's outputs to DIR/*.npy
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 """
 import argparse
@@ -101,12 +102,34 @@ def host_cpu_quota():
     return n
 
 
-def cpu_arm(workload, B, N, warmup, steps, budget_s=None):
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(prob, directory, suffix="", budget=DUMP_BYTES):
+    """--dump-outputs: what the timed path left behind after its last step, i.e. what a caller of to_ilqr_step reads back -- states
+    [B, N, n], controls [B, N-1, m], merit [B] and the accepted step size of the last line search [B] -- as <directory>/<name><suffix>.npy
+    in float64, together with instance_index (the batch rows written).  The inputs are seeded, so two builds run with the same arguments
+    can be compared array for array.  When the batch does not fit in `budget` bytes, a fixed seeded sample of the instances is written,
+    the same rows of every array."""
+    import trajopt_b200 as TO
+    out = {"states": TO.states(prob), "controls": TO.controls(prob), "merit": TO.merit(prob), "step_size": TO.solver_state(prob)["alpha"]}
+    B = prob.B
+    per_instance = sum(a.nbytes for a in out.values()) // B + 8          # + 8: the instance_index entry
+    keep = min(B, (budget - 1024 * (len(out) + 1)) // per_instance)      # 1 KB per file for the .npy headers
+    rows = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    out = {k: v[rows] for k, v in out.items()}
+    out["instance_index"] = rows
+    os.makedirs(directory, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(directory, f"{k}{suffix}.npy"), np.ascontiguousarray(v, dtype=np.float64))
+
+
+def cpu_arm(workload, B, N, warmup, steps, budget_s=None, dump=None):
     """The CPU arm: the oracle port of the same path on the host cores, on the SAME workload as the GPU arm -- the same B instances
     from the same initial state, `warmup` untimed iLQR iterations followed by `steps` timed ones of the same solve (one step = one
     iLQR iteration of every instance).  The warm-up iterations double as the thread-count probe (1x / 2x / 4x the CPU quota, best
     kept).  `budget_s` (cpu_baseline leg of the GPU arm): cap the timed steps so the leg stays near that many seconds -- the steps
-    actually run are reported."""
+    actually run are reported.  `dump`: directory the outputs of the last step go to (dump_outputs)."""
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import oracle_binding as OB
     import trajopt_b200 as TO
@@ -132,6 +155,8 @@ def cpu_arm(workload, B, N, warmup, steps, budget_s=None):
     for _ in range(steps):
         TO.ilqr_step(prob, 1)
     wall = time.perf_counter() - t0
+    if dump:
+        dump_outputs(prob, dump)
     prob.close()
     return {"value": B * steps / wall, "unit": "instance-iterations/s", "cores": nthr, "kind": "port",
             "sample": f"{B} instances x {steps} iLQR iterations after {warmup} warm-up iterations of the same solve as the GPU arm ({wall:.2f} s wall; "
@@ -150,7 +175,7 @@ def run_reference(args, rank, world):
     N = args.N or w["N"]
     per_gpu, glob = batch_split(args, w, world)
     warmup = max(args.warmup, 3)
-    base = cpu_arm(args.workload, glob, N, warmup, args.steps)
+    base = cpu_arm(args.workload, glob, N, warmup, args.steps, dump=args.dump_outputs)
     out = {"impl": "reference", "metric": "ilqr_iterations_per_sec", "value": base["value"], "unit": "instance-iterations/s", "n_gpus": args.gpus,
            "steps": base["steps"], "warmup": warmup, "ms_per_step": base["ms_per_step"], "higher_is_better": True,
            "scaling": args.scaling, "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -195,7 +220,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--e2e-depth", type=int, default=2, help="problem handles in flight in the end-to-end measurement (1 = strictly serial, 2 = double-buffered)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the states, controls, merit and step sizes of the last step to DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
         return run_reference(args, rank, world)
@@ -292,6 +321,8 @@ def main():
     value = B * world * args.steps / (ms * 1e-3)
     st = TO.solver_state(prob)
     accepted_frac = float((st["alpha"] > 0).mean())
+    if args.dump_outputs:   # before the passes below restart the solve on `prob`
+        dump_outputs(prob, args.dump_outputs, f"_rank{rank}" if world > 1 else "", DUMP_BYTES // world)
 
     # ---- per-phase timing pass (CUDA events around each kernel on the launching stream) -> roofline -----------------
     reset()
